@@ -2,6 +2,7 @@
 """bench.py -- MSamples/s of raw I/Q through matched filter -> gate -> tag_decoder.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3|cfg4|cfg5]
+                  [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] ("cfg2"): synthetic 40 kHz-BLF FM0 I/Q @ 2 MS/s, 1000 queries
 (= 1000 inventory-round segments of 16,960 raw samples), 1 tag, per GPU.  One *step* = one pass of the hot path
@@ -15,6 +16,10 @@ Other BASELINE.json configurations (measurement runs; the driver's line stays cf
   cfg3  100,000 inventory rounds in total (1.696e9 raw samples), FIXED_Q=0, sharded over the GPUs ("strong")
   cfg4  FIXED_Q=4: 10,000 rounds x 16 slots = 160,000 slot segments with 8 tags (empty, single and collided slots)
   cfg5  raw-rate sweep 1 / 2 / 4 / 6 / 8 MS/s (decimation 5, ntaps = rate / (2 BLF)): kernel GB/s vs the HBM roofline
+
+--dump-outputs DIR writes what the last timed step computed (window records and counts, see dump_outputs) as
+DIR/<name>.npy; the workload is generated from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference times the reference's own CPU implementation (oracle/_ref: its blocks compiled unchanged, behind
 the canonical matched filter -- GNU Radio's own FIR is not in the reference tree) on all usable host cores over
@@ -49,6 +54,34 @@ CONFIGS = {
                       "(empty, singly occupied and collided slots), per GPU"),
 }
 SWEEP_RATES = [1_000_000, 2_000_000, 4_000_000, 6_000_000, 8_000_000]
+DUMP_BYTES = 60_000_000     # --dump-outputs payload: with the .npy headers below 64 MB however counted
+
+
+def dump_outputs(out_dir, recs, counts, prefix="", extra=None, limit=DUMP_BYTES):
+    """Writes decoded window records (RESULT_DTYPE[nseg, max_windows]) and window counts (int32[nseg]) as
+    out_dir/<prefix><name>.npy: counts.npy and one records_<field>.npy per record field, integer fields as float64,
+    float fields and the bit bytes as float32 (all exact).  `extra` maps names to further per-segment arrays.
+    Above `limit` bytes in all, a fixed seeded sample of the segments is written, their indices in segment_index.npy."""
+    def arrays(sel):
+        out = {"counts": counts[sel].astype(np.float64)}
+        for name in recs.dtype.names:
+            a = recs[name][sel]
+            out["records_" + name] = a.astype(np.float64 if a.dtype.kind == "i" else np.float32)
+        for name, a in (extra or {}).items():
+            out[name] = np.asarray(a)[sel].astype(np.float64)
+        return out
+
+    nseg = counts.size
+    per_seg = sum(a.nbytes for a in arrays(slice(0, 1)).values())
+    if nseg * per_seg <= limit:
+        out = arrays(slice(None))
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(nseg, limit // (per_seg + 8), replace=False))
+        out = arrays(idx)
+        out["segment_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
 
 
 def hbm_peak():
@@ -263,7 +296,13 @@ def main():
     ap.add_argument("--generator", default="torch", choices=["torch", "native"],
                     help="workload generator of our arm (cfg2): the torch model (same samples as the CPU reference arm) or the "
                          "library's CUDA closed-loop slot simulator (rfid_b200_sim_capture)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the window records and counts of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what our timed path computed; the reference arm keeps no records")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.steps is None:
         args.steps = 20 if args.config == "cfg2" else 5
@@ -436,6 +475,12 @@ def main():
     gate1 = check(last % nslots, (args.warmup + last) % len(caps))
     if fixed_q == 0:
         assert gate1["epc_crc_ok"] == nseg and gate1["epc_match_truth"] == nseg, "timed step decoded wrongly: %r" % (gate1,)
+    if args.dump_outputs and rank == 0:
+        # the records every rank holds after the closing all-gather, rank by rank
+        parts = [capi.results_to_numpy(b[last % nslots, : nseg * MAX_WINDOWS],
+                                       b[last % nslots, nseg * MAX_WINDOWS:].view(torch.int32).reshape(-1)[:nseg], MAX_WINDOWS)
+                 for b in (g_block.unbind(0) if world > 1 else (block,))]
+        dump_outputs(args.dump_outputs, np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts]))
 
     # ------------------------------------------------------------------ sampled bit-exact parity against the oracle
     oracle_par = None
@@ -553,22 +598,25 @@ def ingest(args, rank, local_rank):
             segs, recs, counts = rx.ingest_capture_host(iq_np, max_windows=MAX_WINDOWS)
         torch.cuda.synchronize(dev)
         ts = []
-        for _ in range(max(3, args.steps)):
+        for _ in range(args.steps):
             t0 = time.perf_counter()
             segs, recs, counts = rx.ingest_capture_host(iq_np, max_windows=MAX_WINDOWS)
             ts.append(time.perf_counter() - t0)
         t = float(np.median(ts))
+        if args.dump_outputs and kind == "pinned":
+            dump_outputs(args.dump_outputs, recs, counts,
+                         extra={"segments_offset": segs["offset"], "segments_length": segs["length"]})
         ok = int(sum((recs[s, k]["crc_ok"] == 1) for s in range(len(segs)) for k in range(min(int(counts[s]), MAX_WINDOWS)) if recs[s, k]["kind"] == 1))
         rows.append({"host_memory": kind, "seconds_per_call": t, "msamples_per_s": n_raw / t / 1e6, "host_to_device_gbs": 8.0 * n_raw / t / 1e9,
                      "segments_found": int(len(segs)), "epc_crc_ok": ok, "launches_per_call": rx.last_launch_count()})
-    line = {"metric": METRIC, "value": rows[0]["msamples_per_s"], "unit": "MSamples/s", "n_gpus": 1, "steps": max(3, args.steps), "warmup": 2,
+    line = {"metric": METRIC, "value": rows[0]["msamples_per_s"], "unit": "MSamples/s", "n_gpus": 1, "steps": args.steps, "warmup": 2,
             "ms_per_step": rows[0]["seconds_per_call"] * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic",
             "config": {"workload": "ingest: %d-round capture (%.1f MB) in host memory -> segmenter + decode -> host records; wall clock per call, "
                                    "host<->device copies inside" % (rounds, n_raw * 8 / 1e6), "config": "ingest",
                        "hbm_bytes_per_sample": "16 algorithmic (the threshold pass and the decode each read the capture once) + 8 written by the upload"},
             "e2e": {"value": rows[0]["msamples_per_s"], "unit": "MSamples/s", "h2d_bytes_per_step": int(n_raw * 8), "d2h_bytes_per_step": int(rounds * MAX_WINDOWS * 64)},
-            "ingest": rows, "gpu_launches": rows[0]["launches_per_call"] * max(3, args.steps)}
+            "ingest": rows, "gpu_launches": rows[0]["launches_per_call"] * args.steps}
     print(json.dumps(line))
     return 0
 
@@ -606,6 +654,8 @@ def sweep(args, rank, local_rank, world):
         k_ms, k_n = rx.kernel_time(reset=True)
         rx.enable_kernel_timing(False)
         recs, counts = capi.results_to_numpy(res, cnt, MAX_WINDOWS)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, recs, counts, prefix="adc%d_" % adc, limit=DUMP_BYTES // len(SWEEP_RATES))
         ci = (args.warmup + args.steps - 1) % 2
         # parity on a sample of the segments against the oracle at this rate
         pick = np.arange(0, rounds, max(1, rounds // 64))[:64]

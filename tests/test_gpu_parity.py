@@ -10,7 +10,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, records_equal
+from conftest import GOLDEN, load_json, records_equal, ref_segments
 from gen2_uhf_rfid_reader_b200 import abi, synth
 
 pytestmark = pytest.mark.gpu
@@ -28,17 +28,25 @@ def _assert_same(got, ref, what=""):
 
 
 # ------------------------------------------------------------------ cfg1: the reference's own recording
-def test_cfg1_capture_bit_exact_and_readme_stats(rx, cfg1_iq, cfg1_golden):
-    """BASELINE.json configs[0]: misc/data/file_source_test, FIXED_Q=0, as one continuous segment"""
+def _assert_reference_stats(st, g):
+    """READER_STATS of a continuous decode against the reference's run on the same capture"""
+    assert (st.n_queries_sent, st.cur_inventory_round, st.cur_slot_number, st.n_epc_correct) == \
+        (g["n_queries_sent"], g["cur_inventory_round"], g["cur_slot_number"], g["n_epc_correct"])
+    assert st.tag_map() == {int(k): v for k, v in g["tag_reads"].items()}
+
+
+def test_cfg1_capture_bit_exact_and_readme_stats(rx, cfg1_iq, cfg1_golden, cfg1_head_stats):
+    """BASELINE.json configs[0]: misc/data/file_source_test (its first 15 rounds), FIXED_Q=0, as one continuous
+    segment; stats as the reference's print_results on the same samples (README.md:48-53 for the whole file)"""
     recs, counts = rx.decode_capture_host(cfg1_iq, abi.make_segments([0], [cfg1_iq.size]), max_windows=256)
-    assert counts[0] == 142
-    _assert_same(recs[0, :142], cfg1_golden, "cfg1")
-    rel = np.abs(recs[0, :142]["score"] - cfg1_golden["score"]) / cfg1_golden["score"]
+    assert counts[0] == 31
+    _assert_same(recs[0, :31], cfg1_golden, "cfg1")
+    rel = np.abs(recs[0, :31]["score"] - cfg1_golden["score"]) / cfg1_golden["score"]
     assert rel.max() <= 1e-5   # north-star tolerance (actually 0)
     st = rx.reduce_stats(recs, counts, continuous=True)
-    # README.md:48-53
-    assert st.n_queries_sent - 1 == 71 and st.cur_inventory_round == 72 and st.n_epc_correct == 70
-    assert st.tag_map() == {0x27: 70}
+    assert st.n_queries_sent - 1 == 15 and st.cur_inventory_round == 16 and st.n_epc_correct == 14
+    assert st.tag_map() == {0x27: 14}
+    _assert_reference_stats(st, cfg1_head_stats)
 
 
 def test_cfg1_device_resident_call(rx, cfg1_iq, cfg1_golden):
@@ -58,17 +66,17 @@ def test_cfg1_q4_stats(cfg1_iq):
     from gen2_uhf_rfid_reader_b200 import capi
     rx4 = capi.Gen2Rx(fixed_q=4)
     recs, counts = rx4.decode_capture_host(cfg1_iq, abi.make_segments([0], [cfg1_iq.size]), max_windows=256)
-    g = json.load(open(os.path.join(GOLDEN, "cfg1_q4_ref_stats.json")))
-    _assert_same(recs[0, :counts[0]], np.load(os.path.join(GOLDEN, "cfg1_q4_ref_records.npy")), "cfg1 q4")
+    g = load_json("cfg1_q4_head_ref_stats.json")
+    assert counts[0] == g["n_windows"]
+    _assert_same(recs[0, :counts[0]], np.load(os.path.join(GOLDEN, "cfg1_q4_ref_records.npy"))[:g["n_windows"]], "cfg1 q4")
     st = rx4.reduce_stats(recs, counts, continuous=True)
-    assert (st.n_queries_sent, st.cur_inventory_round, st.cur_slot_number, st.n_epc_correct) == \
-        (g["n_queries_sent"], g["cur_inventory_round"], g["cur_slot_number"], g["n_epc_correct"])
+    _assert_reference_stats(st, g)
 
 
 def test_cfg1_segment_slices_with_odd_offsets(rx, oracle, cfg1_iq):
     """rounds cut out of the recording at arbitrary (odd, unaligned) offsets: exercises the 16-byte TMA
     alignment fix-up, partial tiles and the end-of-buffer tail"""
-    offs = [34702 - 1245, 51661 - 801, 68621 - 333, 1247958 - 16961 - 7, 1247958 - 9001]
+    offs = [34702 - 1245, 51661 - 801, 68621 - 333, cfg1_iq.size - 16961 - 7, cfg1_iq.size - 9001]
     lens = [16960, 16961, 16963, 16967, 9001]
     segs = abi.make_segments(offs, lens)
     recs, counts = rx.decode_capture_host(cfg1_iq, segs, max_windows=4)
@@ -92,12 +100,13 @@ def test_synthetic_segments_bit_exact(oracle, kw):
     _assert_same(recs, orecs, str(kw))
 
 
-def test_reference_blocks_agree_on_synthetic(rx, ref_flow):
-    """directly against oracle/_ref (the reference's compiled blocks), not only the restatement"""
+def test_reference_blocks_agree_on_synthetic(rx, ref_outputs):
+    """directly against oracle/_ref (the reference's compiled blocks; tests/golden/reference_outputs.npz), not only the
+    restatement"""
     cap = synth.make_capture(40, seed=5)
     iq = cap["iq"].numpy()
     recs, counts = rx.decode_capture_host(iq, cap["segments"], max_windows=4)
-    rrecs, rcounts, _ = ref_flow.run_segments(iq, cap["segments"], max_per_seg=4)
+    rrecs, rcounts = ref_segments(ref_outputs, 40, 5, {}, iq)
     assert counts.tolist() == rcounts.tolist()
     _assert_same(recs, rrecs, "vs _ref")
 
@@ -116,7 +125,7 @@ def test_ragged_empty_and_tiny_segments(rx, oracle):
 
 
 def test_window_capacity_overflow_counts_but_does_not_store(rx, oracle, cfg1_iq):
-    segs = abi.make_segments([0], [400000])
+    segs = abi.make_segments([0], [cfg1_iq.size])
     recs, counts = rx.decode_capture_host(cfg1_iq, segs, max_windows=3)
     orecs, ocounts, _ = oracle.decode_segments(cfg1_iq, segs, max_per_seg=3)
     assert counts[0] == ocounts[0] > 3
@@ -240,32 +249,42 @@ def test_decode_is_idempotent_and_order_independent(rx):
 
 
 # ------------------------------------------------------------------ the GNU Radio drop-in blocks, end to end
-def test_flowgraph_through_host_blocks_reproduces_readme(cfg1_iq, cfg1_golden):
+def test_flowgraph_through_host_blocks_reproduces_readme(cfg1_iq, cfg1_golden, cfg1_head_stats):
     """apps/reader.py's offline graph with THIS repo's gate / tag_decoder / reader blocks (thin hosts over the
-    C-ABI, GPU underneath) under the oracle's scheduler: README block, records and TX commands as the reference"""
+    C-ABI, GPU underneath) under the oracle's scheduler: README block (the reference's print_results on the same
+    samples), records and TX commands as the reference"""
     import re
-    import sys
     from oracle import refflow
     F = refflow.B200Flow()
     assert not F.is_reference
     r = F.run_stream(cfg1_iq, want_tx=True)
     t = r["text"]
-    for pat, val in ((r"queryreps sent : (\d+)", 71), (r"Inventory round : (\d+)", 72), (r"decoded EPC : (\d+)", 70),
-                     (r"unique tags : (\d+)", 1), (r"Num of reads : (\d+)", 70)):
+    for pat, val in ((r"queryreps sent : (\d+)", 15), (r"Inventory round : (\d+)", 16), (r"decoded EPC : (\d+)", 14),
+                     (r"unique tags : (\d+)", 1), (r"Num of reads : (\d+)", 14)):
         assert int(re.search(pat, t).group(1)) == val, t
+        assert int(re.search(pat, cfg1_head_stats["text"]).group(1)) == val
     assert "Tag ID : 27" in t
-    assert r["n_windows"] == 142
+    assert r["n_windows"] == 31
     _assert_same(r["records"], cfg1_golden, "host blocks")
-    sys.path.insert(0, GOLDEN)
     from make_golden import decode_pie
     cmds = decode_pie(r["tx"])
     gold = json.load(open(os.path.join(GOLDEN, "file_sink_commands.json")))
-    assert [b for k, b in cmds if k == "preamble"][:72] == gold["queries"]
-    assert [b for k, b in cmds if k == "framesync"][:71] == gold["acks"]
+    assert [b for k, b in cmds if k == "preamble"][:16] == gold["queries"][:16] == cfg1_head_stats["tx_queries"]
+    assert [b for k, b in cmds if k == "framesync"][:16] == gold["acks"][:16] == cfg1_head_stats["tx_acks"]
     # chunk-size independent, like the reference
-    r2 = F.run_stream(cfg1_iq[:400000], chunk=257)
-    r3 = F.run_stream(cfg1_iq[:400000], chunk=50000)
+    r2 = F.run_stream(cfg1_iq, chunk=257)
+    r3 = F.run_stream(cfg1_iq, chunk=50000)
     assert r2["records"].tobytes() == r3["records"].tobytes()
+
+
+def test_host_blocks_chunk_size_independent(cfg1_iq, cfg1_golden):
+    """THIS repo's host blocks fed the recording in chunks of any size decode exactly the reference's records (the
+    reference's own blocks give the same records at these chunk sizes: tests/golden/make_golden.py)"""
+    from oracle import refflow
+    F = refflow.B200Flow()
+    for chunk in (257, 4096, 100000):
+        r = F.run_stream(cfg1_iq, chunk=chunk)
+        assert not records_equal(r["records"], cfg1_golden), chunk
 
 
 # ------------------------------------------------------------------ rate sweep (BASELINE.json configs[4])
@@ -320,26 +339,27 @@ def _flatten(recs, counts, segs, decim=5):
 INT_FIELDS = ("open_index", "length", "kind", "sync_index", "crc_ok", "tag_id", "bits", "T")
 
 
-def test_ingest_recording_matches_continuous_reference(rx, cfg1_iq, cfg1_golden):
-    """the reference's own recording, cut at CW gaps by the GPU segmenter and decoded as 72 independent
+def test_ingest_recording_matches_continuous_reference(rx, cfg1_iq, cfg1_golden, cfg1_head_stats):
+    """the reference's own recording, cut at CW gaps by the GPU segmenter and decoded as 16 independent
     segments, reproduces the continuous reference run: every decision bit for bit, scores to the drift of
     the reference's float running means (SURVEY 8e: ~1e-4 relative late in the file)"""
     import segmenter_model as sm
     segs, recs, counts = rx.ingest_capture_host(cfg1_iq, max_windows=4)
     want, cmd = sm.segment_table(cfg1_iq)
     assert [(int(s["offset"]), int(s["length"])) for s in segs] == want
-    assert len(segs) == 72 and counts[:71].tolist() == [2] * 71 and counts[71] == 0   # file ends inside round 72
+    assert len(segs) == 16 and counts[:15].tolist() == [2] * 15 and counts[15] == 1   # capture ends inside round 16's EPC
     assert (segs["offset"] % 5 == 0).all()
     flat = _flatten(recs, counts, segs)
-    assert len(flat) == 142
+    assert len(flat) == 31
     for f in INT_FIELDS:
         assert flat[f].tobytes() == cfg1_golden[f].tobytes(), f
     rel = np.abs(flat["score"] - cfg1_golden["score"]) / cfg1_golden["score"]
     assert rel.max() < 5e-4
     assert np.abs(flat["h_re"] - cfg1_golden["h_re"]).max() < 1e-4 and np.abs(flat["h_im"] - cfg1_golden["h_im"]).max() < 1e-4
     st = rx.reduce_stats(recs, counts, continuous=True)
-    assert st.n_queries_sent - 1 == 71 and st.cur_inventory_round == 72 and st.n_epc_correct == 70   # README.md:48-53
-    assert st.tag_map() == {0x27: 70}
+    assert st.n_queries_sent - 1 == 15 and st.cur_inventory_round == 16 and st.n_epc_correct == 14
+    assert st.tag_map() == {0x27: 14}
+    _assert_reference_stats(st, cfg1_head_stats)
 
 
 def test_ingest_segments_equal_fresh_state_oracle(rx, oracle, cfg1_iq):
@@ -407,28 +427,26 @@ def _script(rn16s):
 
 
 @pytest.mark.parametrize("dac_rate", [1000000, 2000000])
-def test_tx_synth_equals_reference_reader_block(rx, ref_flow, dac_rate):
+def test_tx_synth_equals_reference_reader_block(rx, ref_outputs, dac_rate):
     """the CUDA PIE generator against the reference's own reader block (oracle/_ref), sample for sample"""
-    rng = np.random.default_rng(11)
-    rn16s = rng.integers(0, 65536, size=12)
-    rn16s[0], rn16s[1] = 0x0579, 0xFFFF     # first RN16 of the author's TX capture; all data-1
-    bits = ((rn16s[:, None] >> np.arange(15, -1, -1)[None, :]) & 1).astype(np.float32)
-    want, nq = ref_flow.reader_script(bits, dac_rate=dac_rate)
+    from make_golden import READER_SCRIPTS, rn16_bits, tx_script_rn16s
+    rn16s = tx_script_rn16s()
+    name = "reader_tx_dac%d" % dac_rate
+    assert READER_SCRIPTS[name][2] == dac_rate and np.array_equal(READER_SCRIPTS[name][1], rn16_bits(rn16s))
+    want, nq = ref_outputs[name], int(ref_outputs[name + "_queries"])
     got = rx.tx_synth(_script(rn16s), dac_rate=dac_rate).cpu().numpy()
     assert got.size == want.size and nq == 12
     assert got.tobytes() == want.tobytes()
 
 
-def test_tx_synth_q4_query_crc5_and_other_commands():
+def test_tx_synth_q4_query_crc5_and_other_commands(ref_outputs):
     """FIXED_Q=4 Query (CRC-5 11101, SURVEY App. B) against the q4 reference build; NAK / power-down shapes"""
     from gen2_uhf_rfid_reader_b200 import capi
-    from oracle import refflow
-    if not refflow.ref_available(4):
-        pytest.skip("oracle/_ref q4 build missing")
+    from make_golden import READER_SCRIPTS
     rx4 = capi.Gen2Rx(fixed_q=4)
-    ref4 = refflow.RefFlow(4)
-    bits = np.zeros((2, 16), dtype=np.float32)
-    want, _ = ref4.reader_script(bits)
+    q, bits, dac = READER_SCRIPTS["reader_tx_q4"]
+    assert q == 4 and dac == 1000000 and not bits.any() and bits.shape == (2, 16)
+    want = ref_outputs["reader_tx_q4"]
     got = rx4.tx_synth(_script([0, 0])).cpu().numpy()
     assert got.tobytes() == want.tobytes()
     nak = rx4.tx_synth([(abi.TX_NAK, 0)]).cpu().numpy()

