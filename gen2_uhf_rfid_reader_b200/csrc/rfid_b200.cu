@@ -35,10 +35,11 @@ struct rfid_b200_ctx {
   float* window_tap;
   int last_launches;
   bool timing;
-  cudaEvent_t ev0, ev1;
-  std::vector<std::pair<cudaEvent_t, cudaEvent_t>> pending;
-  std::vector<cudaEvent_t> ev_pool;  // timing events are created once and reused (no driver calls inside a timed loop)
-  float kernel_ms;
+  unsigned long long* d_stamps;      // kernel timing: kStampSlots launch slots {earliest CTA start, latest CTA end} (ns)
+  int stamp_next;                    // slots taken since the last drain
+  cudaStream_t stamp_stream;         // stream of the last timed launch
+  unsigned long long last_end_ns;    // end stamp of the last drained launch
+  double kernel_ms;
   int kernel_launches;
   int sm_count;
   int pack_g_override;  // RFID_B200_PACK_G (developer aid): segments per CTA of the pack kernel, 0 = automatic
@@ -50,7 +51,7 @@ struct rfid_b200_ctx {
   void* d_cnt; size_t d_cnt_bytes;
   void* d_win; size_t d_win_bytes;  // per-segment window scratch of the one-CTA-per-segment kernels
   void* d_yhist;                     // rx_pack_kernel: y history, [%nsmid][kPMaxSeg][kYW] float2
-  cudaEvent_t ev_hist;               // recorded after every rx_pack_kernel launch: the history serves one launch at a time
+  cudaEvent_t ev_hist;               // hist_stream's work, recorded when a launch moves to another stream
   cudaStream_t hist_stream;          // stream of the last rx_pack_kernel launch
   bool hist_used;
   // block mode
@@ -287,18 +288,38 @@ int pack_segments_per_cta(const rfid_b200_ctx* ctx, int nseg)
   return g;
 }
 
-void drain_timing(rfid_b200_ctx* ctx)
+constexpr int kStampSlots = 256;  // timed launches between two drains (a full table is drained before the next launch)
+
+// every slot back to {~0, 0}: stamp_cta_start keeps the minimum, stamp_warp_end the maximum
+cudaError_t reset_stamps(rfid_b200_ctx* ctx)
 {
-  for (auto& pr : ctx->pending) {
-    float ms = 0.f;
-    if (cudaEventSynchronize(pr.second) == cudaSuccess && cudaEventElapsedTime(&ms, pr.first, pr.second) == cudaSuccess) {
-      ctx->kernel_ms += ms;
-      ctx->kernel_launches++;
-    }
-    ctx->ev_pool.push_back(pr.first);
-    ctx->ev_pool.push_back(pr.second);
+  const size_t slot = 2 * sizeof(unsigned long long);
+  cudaError_t e = cudaMemsetAsync(ctx->d_stamps, 0xFF, kStampSlots * slot, ctx->stream);
+  if (e == cudaSuccess) e = cudaMemset2DAsync(ctx->d_stamps + 1, slot, 0, sizeof(unsigned long long), kStampSlots, ctx->stream);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  return e;
+}
+
+// Adds the launches stamped since the last drain to kernel_ms / kernel_launches and frees their slots.  A launch counts
+// the device time it adds to the sequence, end - max(start, previous end): its duration when launches do not overlap,
+// less the part that ran beside the previous launch when they do.
+int drain_timing(rfid_b200_ctx* ctx)
+{
+  if (ctx->stamp_next == 0) return RFID_B200_OK;
+  std::vector<unsigned long long> h(2 * (size_t)ctx->stamp_next);
+  CK(cudaMemcpyAsync(h.data(), ctx->d_stamps, h.size() * sizeof(h[0]), cudaMemcpyDeviceToHost, ctx->stamp_stream));
+  CK(cudaStreamSynchronize(ctx->stamp_stream));
+  for (int i = 0; i < ctx->stamp_next; i++) {
+    const unsigned long long start = h[2 * i], end = h[2 * i + 1];
+    if (end == 0) continue;  // the launch failed
+    const unsigned long long from = std::max(start, ctx->last_end_ns);
+    if (end > from) ctx->kernel_ms += (double)(end - from) * 1e-6;
+    ctx->last_end_ns = std::max(ctx->last_end_ns, end);
+    ctx->kernel_launches++;
   }
-  ctx->pending.clear();
+  ctx->stamp_next = 0;
+  CK(reset_stamps(ctx));
+  return RFID_B200_OK;
 }
 
 }  // namespace
@@ -343,7 +364,8 @@ int rfid_b200_create(const rfid_b200_params* p, rfid_b200_ctx** out)
   rfid_b200_ctx* ctx = new (std::nothrow) rfid_b200_ctx();
   if (!ctx) return RFID_B200_ENOMEM;
   ctx->params = *p; ctx->cfg = cfg; ctx->device = p->device;
-  ctx->window_tap = nullptr; ctx->last_launches = 0; ctx->timing = false; ctx->kernel_ms = 0.f; ctx->kernel_launches = 0;
+  ctx->window_tap = nullptr; ctx->last_launches = 0; ctx->timing = false; ctx->kernel_ms = 0.0; ctx->kernel_launches = 0;
+  ctx->d_stamps = nullptr; ctx->stamp_next = 0; ctx->stamp_stream = nullptr; ctx->last_end_ns = 0;
   ctx->d_iq = ctx->d_segs = ctx->d_res = ctx->d_cnt = ctx->d_in = ctx->d_out = ctx->d_m2 = ctx->d_mf = nullptr;
   ctx->d_win = nullptr; ctx->d_win_bytes = 0;
   ctx->d_yhist = nullptr;
@@ -376,7 +398,8 @@ int rfid_b200_create(const rfid_b200_params* p, rfid_b200_ctx** out)
     init.to_ungate = cfg.len_rn16;
     e = cudaMemcpyAsync(ctx->d_gate, &init, offsetof(GateState, win_samples), cudaMemcpyHostToDevice, ctx->stream);
   }
-  if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&ctx->d_stamps, kStampSlots * 2 * sizeof(unsigned long long));
+  if (e == cudaSuccess) e = reset_stamps(ctx);
   ctx->sm_count = prop.multiProcessorCount;
   {
     const char* ev = getenv("RFID_B200_PACK_G");
@@ -428,11 +451,8 @@ void rfid_b200_destroy(rfid_b200_ctx* ctx)
 {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
-  drain_timing(ctx);
-  for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
-  ctx->ev_pool.clear();
   if (ctx->h_blk) cudaFreeHost(ctx->h_blk);
-  void* ptrs[] = {ctx->d_blk, ctx->d_win, ctx->d_yhist, ctx->d_iq, ctx->d_segs, ctx->d_res, ctx->d_cnt, ctx->d_in, ctx->d_out, ctx->d_m2, ctx->d_mf,
+  void* ptrs[] = {ctx->d_stamps, ctx->d_blk, ctx->d_win, ctx->d_yhist, ctx->d_iq, ctx->d_segs, ctx->d_res, ctx->d_cnt, ctx->d_in, ctx->d_out, ctx->d_m2, ctx->d_mf,
                   ctx->d_gate, ctx->d_gate_out, ctx->d_one, ctx->d_mask, ctx->d_chunk, ctx->d_bursts, ctx->d_ing,
                   ctx->d_script, ctx->d_sim_res, ctx->d_sim_cnt};
   for (void* p : ptrs)
@@ -467,25 +487,18 @@ int rfid_b200_enable_kernel_timing(rfid_b200_ctx* ctx, int on)
 {
   if (!ctx) return RFID_B200_EINVAL;
   ctx->timing = on != 0;
-  if (ctx->timing) {
-    cudaSetDevice(ctx->device);
-    while (ctx->ev_pool.size() < 128) {  // enough for 64 launches in flight before the first drain
-      cudaEvent_t e;
-      if (cudaEventCreate(&e) != cudaSuccess) { cudaGetLastError(); break; }
-      ctx->ev_pool.push_back(e);
-    }
-  }
   return RFID_B200_OK;
 }
 
 int rfid_b200_kernel_time(rfid_b200_ctx* ctx, int reset, float* ms_total, int* launches)
 {
   if (!ctx) return RFID_B200_EINVAL;
-  cudaSetDevice(ctx->device);
-  drain_timing(ctx);
-  if (ms_total) *ms_total = ctx->kernel_ms;
+  CK(cudaSetDevice(ctx->device));
+  const int rc = drain_timing(ctx);
+  if (rc) return rc;
+  if (ms_total) *ms_total = (float)ctx->kernel_ms;
   if (launches) *launches = ctx->kernel_launches;
-  if (reset) { ctx->kernel_ms = 0.f; ctx->kernel_launches = 0; }
+  if (reset) { ctx->kernel_ms = 0.0; ctx->kernel_launches = 0; }
   return RFID_B200_OK;
 }
 
@@ -533,13 +546,14 @@ static int decode_capture_impl(rfid_b200_ctx* ctx, const float* d_iq, size_t n_r
   A.counts = d_counts;
   A.window_tap = reinterpret_cast<float2*>(ctx->window_tap);
   A.cfg = ctx->cfg;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  A.stamps = nullptr;
   if (ctx->timing) {
-    for (cudaEvent_t* pe : {&e0, &e1}) {
-      if (!ctx->ev_pool.empty()) { *pe = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); }
-      else CK(cudaEventCreate(pe));
+    if (ctx->stamp_next == kStampSlots) {
+      int rc = drain_timing(ctx);
+      if (rc) return rc;
     }
-    CK(cudaEventRecord(e0, s));
+    A.stamps = ctx->d_stamps + 2 * ctx->stamp_next++;
+    ctx->stamp_stream = s;
   }
   if (use_pack) {
     PackArgs P;
@@ -547,20 +561,32 @@ static int decode_capture_impl(rfid_b200_ctx* ctx, const float* d_iq, size_t n_r
     make_layout_pack(ctx->cfg, pack_segments_per_cta(ctx, nseg), P);
     P.iq = A.iq; P.n_raw = A.n_raw; P.segs = A.segs; P.nseg = nseg; P.seg_base = seg_base; P.max_windows = A.max_windows;
     P.results = A.results; P.counts = A.counts; P.window_tap = A.window_tap; P.y_hist = reinterpret_cast<float2*>(ctx->d_yhist);
+    P.stamps = A.stamps;
     P.cfg = ctx->cfg;
-    // the y history belongs to one launch at a time: a launch on another stream than the previous one waits for it
-    if (ctx->hist_used && ctx->hist_stream != s) CK(cudaStreamWaitEvent(s, ctx->ev_hist, 0));
-    rx_pack_kernel<5, 5><<<(nseg + P.G - 1) / P.G, 32 * (4 * P.G + 2), P.smem_bytes, s>>>(P);
-    CK(cudaEventRecord(ctx->ev_hist, s));
+    // the y history belongs to one launch at a time: a launch on another stream than the previous one waits for everything
+    // queued on that stream so far (on one stream, each launch completes after the one before it, see rx_pack.cuh)
+    if (ctx->hist_used && ctx->hist_stream != s) {
+      CK(cudaEventRecord(ctx->ev_hist, ctx->hist_stream));
+      CK(cudaStreamWaitEvent(s, ctx->ev_hist, 0));
+    }
+    // programmatic dependent launch: scheduled while the previous kernel of the stream still runs (rx_pack.cuh)
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t lc;
+    memset(&lc, 0, sizeof(lc));
+    lc.gridDim = dim3((nseg + P.G - 1) / P.G);
+    lc.blockDim = dim3(32 * (4 * P.G + 2));
+    lc.dynamicSmemBytes = P.smem_bytes;
+    lc.stream = s;
+    lc.attrs = attr;
+    lc.numAttrs = 1;
+    CK(cudaLaunchKernelEx(&lc, rx_pack_kernel<5, 5>, P));
     ctx->hist_stream = s; ctx->hist_used = true;
   } else {
     fn<<<nseg, fast_path_ok(ctx->cfg) ? kSplitThreads : kFusedThreads, A.smem_bytes, s>>>(A);
   }
   CK(cudaGetLastError());
-  if (ctx->timing) {
-    CK(cudaEventRecord(e1, s));
-    ctx->pending.emplace_back(e0, e1);
-  }
   ctx->last_launches = 1;
   return RFID_B200_OK;
 }

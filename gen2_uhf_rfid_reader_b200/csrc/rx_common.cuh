@@ -270,4 +270,31 @@ __device__ __forceinline__ void named_bar_sync(int id, int nthreads)
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
+// ---- programmatic dependent launch.  A kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may be
+// scheduled while the kernel before it on the stream still runs, as soon as every CTA of that kernel has executed
+// pdl_launch_dependents (or exited).  pdl_wait returns once that kernel has completed and its stores are visible.  In a
+// launch without the attribute both are no-ops.
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+
+// ---- launch timing (rfid_b200_kernel_time).  A launch gets one slot {earliest CTA start, latest CTA end} in %globaltimer
+// ns, reset by the host to {~0, 0}; nullptr = timing off.  Every warp calls stamp_warp_end once, after its last global
+// store; the CTA's last warp stamps the end.  warps_done is a shared counter zeroed before any warp can get there.
+__device__ __forceinline__ unsigned long long global_ns()
+{
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+__device__ __forceinline__ void stamp_cta_start(unsigned long long* slot)
+{
+  if (slot && threadIdx.x == 0) atomicMin(slot, global_ns());
+}
+__device__ __forceinline__ void stamp_warp_end(unsigned long long* slot, unsigned* warps_done)
+{
+  if (!slot) return;
+  __syncwarp();
+  if ((threadIdx.x & 31) == 0 && atomicAdd(warps_done, 1u) == blockDim.x / 32 - 1) atomicMax(slot + 1, global_ns());
+}
+
 }  // namespace rfid_b200

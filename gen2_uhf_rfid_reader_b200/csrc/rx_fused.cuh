@@ -85,6 +85,7 @@ struct FusedArgs {
   int32_t* counts;
   float2* window_tap;            // optional: ungated samples of every stored window (stride len_epc)
   float2* win_scratch;           // [nseg][win_stride]: the window being decoded (RN16 at 0, EPC at rn16_pad); L2-resident
+  unsigned long long* stamps;    // launch timing slot (stamp_cta_start / stamp_warp_end), nullptr = off
   int win_stride, rn16_pad;
   int off_dstage, dstage_samples; // decoder staging buffer
   RxConfig cfg;
@@ -211,6 +212,8 @@ __global__ void __launch_bounds__(kFusedThreads, 8) rx_fused_kernel(const FusedA
 {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ FusedShared B;
+  __shared__ unsigned warps_done;
+  stamp_cta_start(A.stamps);
 
   const int seg = blockIdx.x;
   const int lane = threadIdx.x & 31;
@@ -244,6 +247,7 @@ __global__ void __launch_bounds__(kFusedThreads, 8) rx_fused_kernel(const FusedA
     for (int s = 0; s < kRawStages; s++) mbar_init(&B.raw_full[s], 1);
     for (int s = 0; s < 2; s++) { mbar_init(&B.win_ready[s], 1); mbar_init(&B.win_free[s], 1); }
     B.n_ev = 0;
+    warps_done = 0;
     mbar_fence_init();
   }
   __syncthreads();
@@ -582,6 +586,7 @@ __global__ void __launch_bounds__(kFusedThreads, 8) rx_fused_kernel(const FusedA
       if (lane == 0) mbar_arrive(&B.win_free[j & 1]);
     }
   }
+  stamp_warp_end(A.stamps, &warps_done);
 }
 
 }  // namespace rfid_b200

@@ -209,6 +209,8 @@ __global__ void __launch_bounds__(kSplitThreads, 7) rx_fused_split_kernel(const 
 {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ SplitShared B;
+  __shared__ unsigned warps_done;
+  stamp_cta_start(A.stamps);
 
   const int seg = blockIdx.x;
   const int lane = threadIdx.x & 31;
@@ -270,6 +272,7 @@ __global__ void __launch_bounds__(kSplitThreads, 7) rx_fused_split_kernel(const 
       B.n_ev[s] = 0;
     }
     for (int s = 0; s < 2; s++) { mbar_init(&B.win_ready[s], 1); mbar_init(&B.win_free[s], 1); }
+    warps_done = 0;
     mbar_fence_init();
   }
   __syncthreads();
@@ -873,6 +876,7 @@ __global__ void __launch_bounds__(kSplitThreads, 7) rx_fused_split_kernel(const 
     }
     PH_END(23)
   }
+  stamp_warp_end(A.stamps, &warps_done);
 }
 
 }  // namespace rfid_b200

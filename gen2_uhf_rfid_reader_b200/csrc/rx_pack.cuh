@@ -25,8 +25,15 @@
 //               (rx_decode.cuh); dc_est is subtracted as the decoder reads the samples -- the same exact float
 //               subtraction, gate_impl.cc:173,187.
 //   loader      lane g streams segment g's raw samples through its two half-tile stages as warp A frees them.
-// The history is indexed by the SM (one CTA per SM: the shared-memory request guarantees it), so its size does not depend
-// on the number of segments of the launch; warp A never overwrites a sample a queued window still needs.
+// The history is indexed by the SM (one CTA per SM: the shared-memory request guarantees it, also between two launches
+// that overlap under programmatic dependent launch), so its size does not depend on the number of segments of the launch;
+// warp A never overwrites a sample a queued window still needs.
+// Back-to-back launches overlap (programmatic dependent launch, see DESIGN §4.1): every CTA lets the next launch be
+// scheduled right after the start-up barrier, so the next launch's CTAs take SMs as this launch's CTAs exit.  Before the
+// first store of an output (counts: warp B, records / window tap: warp C) a warp waits for the previous launch to complete,
+// since that launch may write the same buffers; the loader warp waits at its end, so no CTA exits before the previous launch
+// has completed and work queued after a launch still sees every earlier launch.  The inputs (capture, segment table) need no
+// wait: the previous rx_pack_kernel never writes them, and any other kernel before this one has completed when it starts.
 // Shared memory per segment: 2 raw half-tile stages (10 KB), the last dc_length outputs of either half-tile (P1's DC
 // lookback is a lane shuffle plus this tail), a 4-tile ring of |y| (4 KB), the decoder's stage (2 KB); per CTA the
 // running-sum buffers (4 + 5x2 per segment, 1072 B each, skewed so the chain warp's 128-bit accesses are bank-conflict
@@ -48,7 +55,8 @@ constexpr int kPackMaxThreads = 32 * (4 * kPMaxSeg + 2);   // A0, A1, B, C per s
 constexpr int kYW = 4096;                    // samples of y history per segment (power of two)
 constexpr int kPQ = 8;                       // queue of windows that will be decoded (opened, not yet decoded)
 constexpr int kPTrig = 2;                    // windows that may open within one tile (host: len_rn16 >= kT2 / 2)
-constexpr int kPackMinSmem = 116 * 1024;     // request at least this much: two CTAs never share an SM (and its history)
+constexpr int kPackMinSmem = 116 * 1024;     // request at least this much: two CTAs never share an SM (and its history),
+                                             // not even CTAs of two overlapping launches
 
 struct PackArgs {
   const float2* iq;
@@ -61,6 +69,7 @@ struct PackArgs {
   int32_t* counts;
   float2* window_tap;
   float2* y_hist;                            // [%nsmid][kPMaxSeg][kYW]
+  unsigned long long* stamps;                // launch timing slot (stamp_cta_start / stamp_warp_end), nullptr = off
   RxConfig cfg;
   int G;                                     // segments per CTA of this launch
   int raw_stage_samples;
@@ -229,6 +238,8 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ PackSegCtl ctl_all[kPMaxSeg];
   __shared__ PackCtaCtl cta;
+  __shared__ unsigned warps_done;
+  stamp_cta_start(A.stamps);
 #ifdef RFID_B200_PHASE_PROFILE
   __shared__ long long pp_cta_t0;
   if (threadIdx.x == 0) pp_cta_t0 = clock64();
@@ -284,6 +295,7 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
     if (threadIdx.x == 32) {
       for (int s = 0; s < kPAS; s++) { mbar_init(&cta.fullA[s], 2 * G); mbar_init(&cta.avgdone[s], 1); }
       for (int s = 0; s < kPDS; s++) { mbar_init(&cta.p3done[s], G); mbar_init(&cta.dcdone[s], 1); }
+      warps_done = 0;
       mbar_fence_init();
     }
     for (int g = 0; g < G; g++) {
@@ -296,6 +308,8 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
     }
     if (threadIdx.x < G) ctl_all[threadIdx.x].seg = sg0;
     asm volatile("bar.sync 14, %0;" ::"r"((int)blockDim.x) : "memory");   // start-up barrier (the loader joins it below)
+    // the CTA holds its SM: the next launch may be scheduled (it gets SMs as this launch's CTAs exit)
+    pdl_launch_dependents();
     // the CTA's barriers count every warp A / B for every tile of the longest segment
     for (int g = 0; g < g_act; g++) {
       const int n_out_g = (int)(ctl_all[g].seg.length / DECIM);
@@ -544,6 +558,8 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
         __syncwarp();
         if (lane == 0) mbar_arrive(&cta.fullA[i % kPAS]);   // this half of tile i is ready for the chain warp
       }
+      // the next launch's CTA on this SM rewrites the same history: this CTA's history stores are performed before it exits
+      __threadfence();
     } else {
       // ------------------------------------------------------------------------------------- warp B: P3
       // the gate (gate_impl.cc:45, global_vars.cc:47, reader_impl.cc:259,262)
@@ -749,7 +765,8 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
         __syncwarp();
         if (lane == 0) mbar_arrive(&cta.p3done[t % kPDS]);   // the tile's DC list is final
       }
-      // ---- end of the segment
+      // ---- end of the segment (the previous launch may have written the same counts)
+      pdl_wait();
       if (have && lane == 0) A.counts[seg] = B.b_wcount;
       if (lane == 0) { __threadfence_block(); B.seg_done = 1; }
     }
@@ -863,10 +880,13 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
     for (int k = 0; k < 2 && k < nhalf; k++) issue(k);   // both stages are free at the start
     __syncwarp();
     asm volatile("bar.sync 14, %0;" ::"r"((int)blockDim.x) : "memory");   // start-up barrier
+    pdl_launch_dependents();
     for (int k = 2; k < nhalf; k++) {
       mbar_wait_idle(&B.raw_empty[k & 1], (uint32_t)(((k >> 1) - 1) & 1), 100);
       issue(k);
     }
+    // the CTA does not complete before the previous launch has (warps B / C may have stored nothing)
+    pdl_wait();
   } else {
     // ======================================================================================= warp C: decode
     const int g = warp - 3 * G - 2;
@@ -914,6 +934,7 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
         decode_window_staged(C, kind, wv, len, dstage, A.dstage_samples, wd, nullptr, nullptr, dc);
 #endif
         rfid_b200_window_result* dst = A.results + (size_t)seg * A.max_windows + ord;
+        if (k == 0) pdl_wait();   // the previous launch may have written the same records / window tap
         if (lane == 0) store_result(dst, wd, seg + A.seg_base, ord, wopen, len, kind);
 #ifndef RFID_B200_PHASE_PROFILE
         if (A.window_tap) {
@@ -931,6 +952,7 @@ __global__ void __launch_bounds__(kPackMaxThreads, 1) rx_pack_kernel(const PackA
 #endif
     }
   }
+  stamp_warp_end(A.stamps, &warps_done);
 }
 
 }  // namespace rfid_b200

@@ -113,6 +113,8 @@ RFID_B200_API const char* rfid_b200_last_cuda_error(const rfid_b200_ctx* ctx);
 RFID_B200_API void rfid_b200_default_params(rfid_b200_params* p);
 
 /* Context: one per block instance (block mode) or per decode stream (capture mode).
+ * A capture-mode call on another stream than the context's previous one waits for
+ * everything queued on that previous stream, which must therefore still exist.
  * Replaces the constructors gate_impl.cc:41-70 / tag_decoder_impl.cc:50-62 and the
  * process-global reader_state (global_vars.cc:34-54). */
 RFID_B200_API int rfid_b200_create(const rfid_b200_params* p, rfid_b200_ctx** out);
@@ -147,8 +149,11 @@ RFID_B200_API int rfid_b200_decode_capture_host(rfid_b200_ctx* ctx, const float*
 
 /* Kernel launches issued by the last decode_capture call on this context. */
 RFID_B200_API int rfid_b200_last_launch_count(const rfid_b200_ctx* ctx);
-/* Device time (ms, CUDA events on the launch stream) of the dominant kernel
- * (fused matched-filter+gate) accumulated since the last reset; and its launches. */
+/* Device time (ms) of the decode kernel accumulated since the last reset, and its
+ * launches, while timing is enabled.  Each launch stamps its first CTA start and
+ * last CTA end on the GPU's global timer and counts end - max(start, end of the
+ * previous launch): the device time it adds to a back-to-back sequence, without
+ * launch latency.  Synchronises with the stream of the last timed launch. */
 RFID_B200_API int rfid_b200_kernel_time(rfid_b200_ctx* ctx, int reset, float* ms_total, int* launches);
 RFID_B200_API int rfid_b200_enable_kernel_timing(rfid_b200_ctx* ctx, int on);
 
